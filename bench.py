@@ -32,6 +32,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 
@@ -53,7 +54,13 @@ def parse_args():
     ap.add_argument("--conv-tf32", action="store_true", help="let the retained cuDNN convs use TF32 (reference GPU default)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-points", type=int, default=262144, help="points of the CPU-baseline tile")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (train: loss, gradients, updated "
+                         "parameters; infer: the summed height and weight rasters), a fixed sample of it beyond 60 MB")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 def synthetic_batch(tiles, points, seed, with_image=False):
@@ -61,6 +68,23 @@ def synthetic_batch(tiles, points, seed, with_image=False):
     cloud = synthetic_cloud(tiles, points, seed, clustered=True)
     dsm, image = synthetic_targets(tiles, 512, seed, with_image=with_image)
     return cloud, dsm, image
+
+
+DUMP_BYTES = 60 << 20  # array data of --dump-outputs: the .npy files stay under 64 MB together
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every name -> float32 / float64 CPU tensor as out_dir/<name>.npy.  When they hold more than DUMP_BYTES
+    together, every array of more than one element is cut to the same fraction of its flat elements, taken in order
+    at positions drawn from a fixed seed: runs with the same arguments store the same elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() * t.element_size() for t in arrays.values())
+    for name, t in arrays.items():
+        assert t.dtype in (torch.float32, torch.float64), (name, t.dtype)
+        if total > DUMP_BYTES and t.numel() > 1:
+            pos = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:t.numel() * DUMP_BYTES // total]
+            t = t.flatten()[pos.sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
 
 
 def load_peaks():
@@ -264,7 +288,7 @@ def build_model(cfg, dev, seed=0):
     return t2h.TomoSAR2Height(cfg).to(dev)
 
 
-def run_train(args, ctx, use_image, tiles, steps, warmup, want_kernels):
+def run_train(args, ctx, use_image, tiles, steps, warmup, want_kernels, want_outputs=False):
     import tomosar2height_b200 as t2h
     from tomosar2height_b200 import _lib
     from tomosar2height_b200.trainer import Trainer
@@ -299,6 +323,9 @@ def run_train(args, ctx, use_image, tiles, steps, warmup, want_kernels):
            "points": ctx.world * tiles * N * steps, "px": ctx.world * tiles * 512 * 512 * steps,
            "h2d": sum(t.numel() * t.element_size() for t in host), "d2h": 4,
            "grad_bytes": trainer.flat.nbytes, "allreduce_ms": trainer.last_allreduce_ms()}
+    if want_outputs:  # taken before the kernel-timing step below moves the model on
+        res["outputs"] = {"loss": torch.tensor(last, dtype=torch.float32), "gradients": trainer.flat.flat.cpu(),
+                          "parameters": torch.cat([p.detach().flatten() for p in model.parameters()]).cpu()}
     if want_kernels:
         # per-kernel device times (roofline): the same step issued eagerly with CUDA events around every C-ABI call --
         # a graph replay has no host-visible launch boundaries; kernel durations are the same
@@ -333,7 +360,7 @@ def munich_scene(scale, dev, seed=0):
     return pts, lo, (lo[0] + W, lo[1] + H)
 
 
-def run_infer(args, ctx, scale, steps, warmup):
+def run_infer(args, ctx, scale, steps, warmup, want_outputs=False):
     import tomosar2height_b200 as t2h
     from tomosar2height_b200.generator import SceneGenerator
     dev = ctx.dev
@@ -358,10 +385,13 @@ def run_infer(args, ctx, scale, steps, warmup):
         step_resident()
     ms, _ = ctx.timed(step_resident, steps)
     ms_e2e, out = ctx.timed(step_e2e, steps)
-    return {"ms": ms, "ms_e2e": ms_e2e, "points": pts_d.shape[0] * steps, "px": gen.n_rows * gen.n_cols * steps,
-            "tiles": len(gen.anchors), "scene_m": [hi[0] - lo[0], hi[1] - lo[1]], "scene_points": pts_d.shape[0],
-            "h2d": pts_h.numel() * 8, "d2h": getattr(step_e2e, "d2h", 0),
-            "covered_fraction": float((out[1] > 0).double().mean()) if out is not None else None}
+    res = {"ms": ms, "ms_e2e": ms_e2e, "points": pts_d.shape[0] * steps, "px": gen.n_rows * gen.n_cols * steps,
+           "tiles": len(gen.anchors), "scene_m": [hi[0] - lo[0], hi[1] - lo[1]], "scene_points": pts_d.shape[0],
+           "h2d": pts_h.numel() * 8, "d2h": getattr(step_e2e, "d2h", 0),
+           "covered_fraction": float((out[1] > 0).double().mean()) if out is not None else None}
+    if want_outputs:
+        res["outputs"] = {"dsm_sum": out[0], "weight_sum": out[1]}
+    return res
 
 
 def roofline_of(kernels, ms_step):
@@ -407,7 +437,8 @@ def run_b200(args):
     wl = args.workload
     extras = {}
     if wl in ("train", "train_image"):
-        res = run_train(args, ctx, wl == "train_image", args.tiles, args.steps, args.warmup, want_kernels=True)
+        res = run_train(args, ctx, wl == "train_image", args.tiles, args.steps, args.warmup, want_kernels=True,
+                        want_outputs=bool(args.dump_outputs))
         ms_step = res["ms"] / args.steps
         line = {
             "metric": "fwd+bwd points/s", "value": res["points"] / (res["ms"] / 1e3), "unit": "points/s", "n_gpus": world,
@@ -425,7 +456,7 @@ def run_b200(args):
             "gpu_launches": res["launches"], "clocks": res["clocks"], "roofline": roofline_of(res["kernels"], ms_step),
             "kernels": {k: {kk: round(vv, 4) if isinstance(vv, float) else vv for kk, vv in v.items()} for k, v in res["kernels"].items()},
         }
-        cfg, model = res["cfg"], res["model"]
+        cfg, model, outputs = res["cfg"], res["model"], res.get("outputs")
         if wl == "train" and not args.no_extras:
             # configs 3 and 4 on bounded samples, so that the driver's BENCH / SCALE records carry them too
             del res
@@ -445,7 +476,8 @@ def run_b200(args):
                           f"tile list split over {world} GPU(s), 2 passes after 3 warm-ups"}
             line["workloads"] = extras
     else:
-        res = run_infer(args, ctx, args.scene_scale, args.steps, args.warmup)
+        res = run_infer(args, ctx, args.scene_scale, args.steps, args.warmup, want_outputs=bool(args.dump_outputs))
+        outputs = res.get("outputs")
         line = {
             "metric": "scene points/s", "value": res["points"] / (res["ms"] / 1e3), "unit": "points/s", "n_gpus": world,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": res["ms"] / args.steps, "higher_is_better": True,
@@ -482,6 +514,8 @@ def run_b200(args):
             loss_gpu = torch.nn.functional.l1_loss(pa_gpu.squeeze(), d1.to(ctx.dev).squeeze()).item()
             line["parity"] = {"tile_points": n_cpu, "heights_rel": float((pa_gpu.cpu() - pa_cpu).abs().max() / pa_cpu.abs().max()),
                               "loss_rel": abs(loss_gpu - loss_cpu) / abs(loss_cpu), "tolerance": 1e-4}
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         ctx.dist.destroy_process_group()

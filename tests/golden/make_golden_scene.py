@@ -81,6 +81,11 @@ def main():
     for tag, shape, hb in (("w128", (128, 128), [0.5, 0.5]), ("w512", (512, 512), [0.5, 0.5]), ("w9x7", (9, 7), [0.3, 0.5]),
                            ("w16", (16, 16), [0.0, 0.25])):
         out["window_" + tag] = DSMGenerator._linear_blend_patch_weight(shape, hb).numpy()
+    # the 512 x 512 window is kept as its two ramps (row and column 255, where the other ramp is 1): their outer product
+    # is the window bit for bit, and the file stays small
+    w = out.pop("window_w512")
+    out["window_w512_wy"], out["window_w512_wx"] = w[:, 255].copy(), w[255].copy()
+    assert np.array_equal(np.outer(out["window_w512_wy"], out["window_w512_wx"]), w)
     # ---- crop + normalise (crop_cloud.py:21-29, dataset.py:185-196,243-278) ----------------------------------
     g = torch.Generator().manual_seed(21)
     lo = torch.tensor([386000.0, 5820000.0], dtype=torch.float64)

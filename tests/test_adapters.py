@@ -1,15 +1,11 @@
-"""Config / IO adapters (f4): the Hydra-free loader against the reference's conf/ tree (a replica of its structure
-when /root/reference is not mounted), the chunk reader and the raster container."""
-import os
-
+"""Config / IO adapters (f4): the Hydra-free loader against a replica of the structure of the reference's conf/
+tree, the chunk reader and the raster container."""
 import numpy as np
 import pytest
 import yaml
 
 import tomosar2height_b200 as t2h
 from tomosar2height_b200.adapters import ChunkCloud, load_config, read_raster, write_raster
-
-REF_CONF = "/root/reference/conf"
 
 
 def _replica(tmp_path):
@@ -37,11 +33,9 @@ def _replica(tmp_path):
     return str(conf)
 
 
-@pytest.mark.parametrize("source", ["replica", "reference"])
+@pytest.mark.parametrize("source", ["replica"])
 def test_load_config_composes_like_hydra(tmp_path, source):
-    if source == "reference" and not os.path.isdir(REF_CONF):
-        pytest.skip("/root/reference is not mounted")
-    conf = REF_CONF if source == "reference" else _replica(tmp_path)
+    conf = _replica(tmp_path)
     cfg = load_config(conf)  # defaults: model tomosar2height, dataset munich
     assert cfg.dataset.name == "munich" and cfg.use_footprint is True
     assert cfg.model.encoder_kwargs.unet_kwargs.depth == 6                      # munich.yaml overrides the model group

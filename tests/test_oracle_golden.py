@@ -113,9 +113,11 @@ def test_scene_pieces_match_reference(golden_dir):
     import math
     from oracle.generator import blend_window, crop_normalize_tile, raster_col_row, accumulate_scene
     v = np.load(os.path.join(golden_dir, "scene_vectors.npz"))
+    ref_windows = {tag: v["window_" + tag] for tag in ("w128", "w9x7", "w16")}
+    ref_windows["w512"] = np.outer(v["window_w512_wy"], v["window_w512_wx"])  # stored as its two ramps: same bits
     for tag, shape, hb in (("w128", (128, 128), (0.5, 0.5)), ("w512", (512, 512), (0.5, 0.5)), ("w9x7", (9, 7), (0.3, 0.5)),
                            ("w16", (16, 16), (0.0, 0.25))):
-        assert np.array_equal(blend_window(*shape, hb).numpy(), v["window_" + tag]), tag
+        assert np.array_equal(blend_window(*shape, hb).numpy(), ref_windows[tag]), tag
     pts = torch.from_numpy(v["crop_points"])
     for k in range(2):
         x0, y0 = v[f"crop_anchor_{k}"]

@@ -5,6 +5,7 @@ contiguous fp32 CUDA tensor, a RuntimeError is raised.
 """
 import ctypes
 import os
+import shutil
 import subprocess
 import threading
 
@@ -85,8 +86,15 @@ _lock = threading.Lock()
 launch_count = 0  # kernels-launching C calls made through this binding (bench.py reports it)
 
 
+def _nvcc() -> str:
+    """nvcc from PATH, else from the CUDA toolkit named by CUDA_HOME / CUDA_PATH (default /usr/local/cuda)."""
+    home = os.environ.get("CUDA_HOME") or os.environ.get("CUDA_PATH") or "/usr/local/cuda"
+    return shutil.which("nvcc") or os.path.join(home, "bin", "nvcc")
+
+
 def build_library(verbose: bool = False) -> str:
-    """Compile csrc/*.cu for sm_100a into libt2h.so (in-tree, so it travels with the snapshot)."""
+    """Compile csrc/*.cu for sm_100a into libt2h.so (in-tree, next to the package that loads it)."""
+    nvcc = _nvcc()
     build_dir = os.path.join(_ROOT, "build")
     os.makedirs(build_dir, exist_ok=True)
     objects = []
@@ -100,7 +108,7 @@ def build_library(verbose: bool = False) -> str:
         objects.append(obj)
         if os.path.exists(obj) and os.path.getmtime(obj) > max(os.path.getmtime(src_path), newest_header):
             continue
-        cmd = ["nvcc", *NVCC_FLAGS, "-I", os.path.join(_ROOT, "include"), "-I", CSRC, "-c", src_path, "-o", obj]
+        cmd = [nvcc, *NVCC_FLAGS, "-I", os.path.join(_ROOT, "include"), "-I", CSRC, "-c", src_path, "-o", obj]
         if verbose:
             print(" ".join(cmd))
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
@@ -110,7 +118,7 @@ def build_library(verbose: bool = False) -> str:
             raise RuntimeError(f"nvcc failed for {src}:\n{out}")
     stale = not os.path.exists(LIB_PATH) or any(os.path.getmtime(o) > os.path.getmtime(LIB_PATH) for o in objects)
     if procs or stale:
-        cmd = ["nvcc", "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", LIB_PATH, *objects]
+        cmd = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", LIB_PATH, *objects]
         res = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
         if res.returncode != 0:
             raise RuntimeError(f"link failed:\n{res.stdout}")
