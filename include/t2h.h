@@ -258,6 +258,15 @@ int t2h_tile_write(const double* points, const void* items, int64_t n_items, con
 int t2h_blend_accumulate(const float* heights, int n_tiles, int S, const int32_t* t_row, const int32_t* l_col,
                          const double* wx, const double* wy, int r0, int c0, int box_rows, int box_cols, int n_rows,
                          int n_cols, double* dsm, double* weight, t2h_stream_t stream);
+/* orthophoto windows of a tile batch (models with the image branch, model.py:54-67), cut from a planar float32 scene
+ * raster (C, rows, cols) that stays on the device:
+ *   out[b, h, j, c] = (raster[c, t_row[b] + S-1-h, l_col[b] + j] - mean[c]) / std[c]     (fp32 subtraction, IEEE division)
+ * `out` is channels-last (B, S, S, C), the image encoder's (B, C, S, S) input.  Window row h is raster row t_row + S-1-h,
+ * the flip of t2h_blend_accumulate: row 0 is the southern edge, like row 0 of the cloud plane (pixel.py:105-111 adds the
+ * two planes pixel by pixel).  Pixels outside the raster are written as NaN. */
+int t2h_raster_windows(const float* raster, int C, int64_t rows, int64_t cols, const int32_t* t_row,
+                       const int32_t* l_col, int n_tiles, int S, const float* mean, const float* std_dev, float* out,
+                       t2h_stream_t stream);
 
 /* bias gradient: out[c] = sum_r g[r, c], two-stage and deterministic */
 size_t t2h_colsum_workspace_bytes(int64_t rows, int n);

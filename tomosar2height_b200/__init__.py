@@ -13,7 +13,7 @@ from .config import berlin_config, munich_config, Config, to_config  # noqa: F40
 from .topology import RaggedCloud  # noqa: F401
 from .adapters import load_config, ChunkCloud, write_raster, read_raster  # noqa: F401
 from .trainer import Trainer  # noqa: F401
-from .generator import SceneGenerator  # noqa: F401
+from .generator import SceneGenerator, OrthoImage  # noqa: F401
 
 
 def install_as_reference():

@@ -47,6 +47,7 @@ SIGNATURES = {
     "t2h_tile_count": [_p, _p, _i64, _p, _f64, _p, _p, _p],
     "t2h_tile_write": [_p, _p, _i64, _p, _f64, _f64, _p, _p, _p, _p],
     "t2h_blend_accumulate": [_p, _i32, _i32, _p, _p, _p, _p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _p],
+    "t2h_raster_windows": [_p, _i32, _i64, _i64, _p, _p, _i32, _i32, _p, _p, _p, _p],
     "t2h_upsample_bilinear_fwd": [_p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p],
     "t2h_upsample_bilinear_bwd": [_p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p],
     "t2h_split_tf32": [_p, _i64, _p, _p, _p],

@@ -1,5 +1,6 @@
 // Scene inference either side of the model forward (SURVEY §8f rank f2): tile crop + normalisation of the
-// binned scene cloud, and flip * blend-window * accumulate of the predicted tiles into the scene rasters.
+// binned scene cloud, the normalised orthophoto windows of the tiles (models with the image branch), and
+// flip * blend-window * accumulate of the predicted tiles into the scene rasters.
 //
 // Replace, per tile, the CPU boolean mask over a whole chunk (dataset.py:234 -> utils/crop_cloud.py:21-29),
 // the 4x4 normalisation matmul + float cast + re-crop (dataset.py:243-278) and the python slice-add of
@@ -146,6 +147,32 @@ blend_accumulate_kernel(const float* __restrict__ heights, int n_tiles, int S, c
   }
 }
 
+// out[b, h, j, c] = (raster[c, t_row[b] + S-1-h, l_col[b] + j] - mean[c]) / std[c], channels-last (B, S, S, C).
+// Row h of a window is raster row t_row + S-1-h: the same flip as blend_accumulate applies to the heights, so that
+// window row 0 is the southern edge like row 0 of the cloud plane (y cell index).  A plain fp32 subtraction and an
+// IEEE division, bitwise equal to the torch expression.  Pixels outside the raster are written as NaN (the caller
+// checks coverage on the host; this only keeps a bad origin from reading out of bounds).
+// One block row per output row (b, h), threads over j: every channel plane is read with coalesced loads, and the
+// C interleaved stores of a warp cover one contiguous 128*C-byte run.
+constexpr int kWindowThreads = 128;
+
+__global__ void __launch_bounds__(kWindowThreads)
+raster_windows_kernel(const float* __restrict__ raster, int C, int64_t rows, int64_t cols,
+                      const int32_t* __restrict__ t_row, const int32_t* __restrict__ l_col, int S,
+                      const float* __restrict__ mean, const float* __restrict__ std_dev, float* __restrict__ out) {
+  const int bh = blockIdx.x;  // b * S + h
+  const int b = bh / S, h = bh - b * S;
+  const int j = blockIdx.y * kWindowThreads + threadIdx.x;
+  if (j >= S) return;
+  const int64_t r = (int64_t)t_row[b] + (S - 1 - h), c = (int64_t)l_col[b] + j;
+  const bool inside = r >= 0 && r < rows && c >= 0 && c < cols;
+  const int64_t plane = rows * cols;
+  const float* src = raster + r * cols + c;
+  float* dst = out + ((int64_t)bh * S + j) * C;
+  for (int ch = 0; ch < C; ++ch)
+    dst[ch] = inside ? __fdiv_rn(__fsub_rn(src[ch * plane], mean[ch]), std_dev[ch]) : __int_as_float(0x7fc00000);
+}
+
 }  // namespace t2h
 
 using namespace t2h;
@@ -185,6 +212,21 @@ extern "C" int t2h_blend_accumulate(const float* heights, int n_tiles, int S, co
   if (n_tiles == 0 || px == 0) return T2H_OK;
   blend_accumulate_kernel<<<(unsigned)((px + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       heights, n_tiles, S, t_row, l_col, wx, wy, r0, c0, box_rows, box_cols, n_rows, n_cols, dsm, weight);
+  T2H_CHECK_LAUNCH();
+  return T2H_OK;
+}
+
+extern "C" int t2h_raster_windows(const float* raster, int C, int64_t rows, int64_t cols, const int32_t* t_row,
+                                  const int32_t* l_col, int n_tiles, int S, const float* mean, const float* std_dev,
+                                  float* out, t2h_stream_t stream) {
+  if (C <= 0 || rows <= 0 || cols <= 0 || n_tiles < 0 || S <= 0 ||
+      (n_tiles > 0 && (!raster || !t_row || !l_col || !mean || !std_dev || !out)))
+    return T2H_ERR_INVALID_ARGUMENT;
+  if ((int64_t)n_tiles * S > 0x7fffffff) return T2H_ERR_UNSUPPORTED_SHAPE;
+  if (n_tiles == 0) return T2H_OK;
+  const dim3 grid((unsigned)(n_tiles * S), (unsigned)((S + kWindowThreads - 1) / kWindowThreads));
+  raster_windows_kernel<<<grid, kWindowThreads, 0, (cudaStream_t)stream>>>(raster, C, rows, cols, t_row, l_col, S,
+                                                                          mean, std_dev, out);
   T2H_CHECK_LAUNCH();
   return T2H_OK;
 }

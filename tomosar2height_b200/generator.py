@@ -9,12 +9,56 @@ candidates from <= 9 contiguous cell ranges instead of scanning the whole chunk 
 (dataset.py:234), and tiles with different point counts are batched as a ``RaggedCloud``.
 No collective is needed: with several GPUs every rank generates a block of the tile list into its own
 partial rasters (``tile_range``), which are summed afterwards.
+Models with the image branch get, per batch, the normalised orthophoto windows of the tiles, cut on the device
+from an ``OrthoImage`` that stays resident (t2h_raster_windows).
 """
 import math
 
+import numpy as np
 import torch
 
 from .topology import RaggedCloud
+
+
+class OrthoImage:
+    """An orthophoto on the device, the image input of scene generation.
+
+    ``bands`` (C, H, W) float32, row 0 = northern edge (the layout of ``read_raster`` / ``write_raster``); ``left``,
+    ``top`` the world coordinates of its upper-left corner and ``pixel_size`` its (square) pixel edge; ``mean`` /
+    ``std`` the per-channel normalisation of the training images (dataset.py:111-113): a window is fed to the model as
+    (band - mean) / std."""
+
+    def __init__(self, bands, left, top, pixel_size, mean, std, device="cuda"):
+        if not isinstance(bands, torch.Tensor):
+            bands = np.asarray(bands)
+            if bands.dtype != np.float32:
+                raise ValueError(f"OrthoImage: bands must be float32, got {bands.dtype}")
+            bands = torch.from_numpy(bands)
+        elif bands.dtype != torch.float32:
+            raise ValueError(f"OrthoImage: bands must be float32, got {bands.dtype}")
+        if bands.dim() != 3:
+            raise ValueError(f"OrthoImage: bands must be (C, H, W), got shape {tuple(bands.shape)}")
+        C = bands.shape[0]
+        mean = torch.as_tensor(mean, dtype=torch.float32).flatten()
+        std = torch.as_tensor(std, dtype=torch.float32).flatten()
+        if mean.numel() != C or std.numel() != C:
+            raise ValueError(f"OrthoImage: mean and std need {C} values (one per band), got {mean.numel()} and {std.numel()}")
+        if bool((std == 0).any()):
+            raise ValueError("OrthoImage: std must not be 0")
+        self.bands = bands.to(device).contiguous()
+        self.left, self.top, self.pixel_size = float(left), float(top), float(pixel_size)
+        self.mean, self.std = mean.to(device), std.to(device)
+
+    @classmethod
+    def from_raster(cls, path, mean, std, device="cuda"):
+        """Read a ``write_raster`` container (``path.npy`` + ``path.json``): corner and pixel size from its affine
+        (px, 0, left, 0, -px, top)."""
+        from .adapters import read_raster
+        bands, meta = read_raster(path)
+        a, b, left, d, e, top = meta["transform"]
+        if b != 0.0 or d != 0.0 or a != -e:
+            raise ValueError(f"OrthoImage.from_raster: {path} is rotated or has non-square pixels ({meta['transform']})")
+        return cls(bands, left, top, a, mean, std, device)
 
 
 def regular_anchors(lo, hi, patch, stride):
@@ -166,20 +210,49 @@ class SceneGenerator:
                   _lib.ptr(item_offset), _lib.ptr(zmin), _lib.ptr(out))
         return out, counts
 
-    def raster_window(self, x0, y0):
-        """generator.py:139-154 with RasterData.query_col_row (io_raster.py:123-131): (t_row, l_col) of a tile."""
-        l_col = math.floor((x0 + self.px / 2 - self.l) / self.px)
-        t_row = math.floor((self.t - (y0 + self.patch - self.px / 2)) / self.px)
+    def raster_window(self, x0, y0, left=None, top=None):
+        """generator.py:139-154 with RasterData.query_col_row (io_raster.py:123-131): (t_row, l_col) of a tile in the
+        output raster, or in a raster of the same pixel size whose upper-left corner is (left, top)."""
+        left = self.l if left is None else left
+        top = self.t if top is None else top
+        l_col = math.floor((x0 + self.px / 2 - left) / self.px)
+        t_row = math.floor((top - (y0 + self.patch - self.px / 2)) / self.px)
         return t_row, l_col
 
+    def _check_inputs(self, points, image):
+        """Host-side checks of the modalities and the orthophoto, before anything is launched."""
+        use_image = bool(getattr(self.model, "use_image", False))
+        if use_image and image is None:
+            raise ValueError("generate: the model has the image branch (use_image); pass image=OrthoImage(...)")
+        if image is None:
+            return
+        if not use_image:
+            raise ValueError("generate: an image was passed but the model has no image branch (use_image is false)")
+        if image.pixel_size != self.px:
+            raise ValueError(f"generate: image pixel size {image.pixel_size} != output pixel size {self.px}")
+        C, H, W = image.bands.shape
+        if C != self.model.image_encoder.in_channels:
+            raise ValueError(f"generate: image has {C} bands, the image encoder takes {self.model.image_encoder.in_channels}")
+        if image.bands.device != points.device:
+            raise ValueError(f"generate: image on {image.bands.device}, points on {points.device}")
+        S = int(round(self.patch / self.px))
+        for x0, y0 in self.anchors:
+            t_row, l_col = self.raster_window(x0, y0, image.left, image.top)
+            if t_row < 0 or l_col < 0 or t_row + S > H or l_col + S > W:
+                raise ValueError(f"generate: the image ({H} x {W} pixels from ({image.left}, {image.top})) does not cover "
+                                 f"the tile at ({x0}, {y0}): window rows {t_row}..{t_row + S - 1}, columns {l_col}..{l_col + S - 1}")
+
     @torch.no_grad()
-    def generate(self, points, tile_range=None, rank=None, world=None):
-        """points (P, 3) world coordinates on the device (float64 recommended for geo-coordinates).
+    def generate(self, points, image=None, tile_range=None, rank=None, world=None):
+        """points (P, 3) world coordinates on the device (float64 recommended for geo-coordinates); ``image`` an
+        ``OrthoImage`` on the same device, required by models with the image branch (tiles without points are skipped
+        whatever the modality, as the dataset marks them invalid: dataset.py:235-241).
         Returns (dsm (n_rows, n_cols) float64, weight float64); with ``tile_range`` (or ``rank`` / ``world``: a
         contiguous block of the tile list balanced by candidate points, identical on every rank without
         communication) the un-normalised partial sums of that block of tiles -- sum the partials of all ranks, then
         ``finalize``."""
         from . import _lib
+        self._check_inputs(points, image)
         dev = points.device
         if tile_range is None and world is not None:
             binned, tile_range = self._bin(points.double(), rank, world)
@@ -202,6 +275,14 @@ class SceneGenerator:
         t_rows = torch.tensor([w[0] for w in win], dtype=torch.int32, device=dev)
         l_cols = torch.tensor([w[1] for w in win], dtype=torch.int32, device=dev)
         bounds = torch.tensor([starts[t] for t in live] + [0], dtype=torch.int64, device=dev)
+        if image is not None:
+            # the tiles' orthophoto windows: the same arithmetic on the image's own corner
+            img_win = [self.raster_window(*todo[t], image.left, image.top) for t in live]
+            img_rows = torch.tensor([w[0] for w in img_win], dtype=torch.int32, device=dev)
+            img_cols = torch.tensor([w[1] for w in img_win], dtype=torch.int32, device=dev)
+            C, H, W = image.bands.shape
+            windows = torch.empty(self.tiles_per_batch, S, S, C, dtype=torch.float32, device=dev)
+        use_cloud = bool(getattr(self.model, "use_cloud", True))
         self.model.eval()
         for k in range(0, len(live), self.tiles_per_batch):
             tiles = live[k:k + self.tiles_per_batch]
@@ -209,7 +290,13 @@ class SceneGenerator:
             p0, p1 = starts[tiles[0]], starts[tiles[-1]] + counts[tiles[-1]]
             # live tiles are contiguous in the flat buffer (empty ones hold no rows); offsets relative to the batch
             offsets = torch.cat([bounds[k:k + nb] - p0, bounds.new_tensor([p1 - p0])])
-            heights = self.model(input_cloud=RaggedCloud(flat[p0:p1], offsets))[0]  # (B, S, S, 1)
+            cloud = RaggedCloud(flat[p0:p1], offsets) if use_cloud else None
+            img = None
+            if image is not None:
+                _lib.call("t2h_raster_windows", _lib.ptr(image.bands), C, H, W, _lib.ptr(img_rows[k:k + nb]),
+                          _lib.ptr(img_cols[k:k + nb]), nb, S, _lib.ptr(image.mean), _lib.ptr(image.std), _lib.ptr(windows))
+                img = windows[:nb].permute(0, 3, 1, 2)  # channels-last memory, the NCHW view the image encoder takes
+            heights = self.model(input_cloud=cloud, input_image=img)[0]  # (B, S, S, 1)
             rows = [w[0] for w in win[k:k + nb]]
             cols = [w[1] for w in win[k:k + nb]]
             r0, c0 = min(rows), min(cols)
