@@ -268,6 +268,20 @@ int t2h_raster_windows(const float* raster, int C, int64_t rows, int64_t cols, c
                        const int32_t* l_col, int n_tiles, int S, const float* mean, const float* std_dev, float* out,
                        t2h_stream_t stream);
 
+/* ---- evaluation of a scene nDSM against the ground-truth DSM (evaluator.py:53-99: residual statistics per mask class,
+ *      evaluator.py:83-95).  A pixel is valid when pred and gt are finite and (use_nodata) gt != nodata; r = pred - gt
+ *      (one fp64 subtraction).  Class 0 is every valid pixel, class c + 1 the valid pixels with bit c of
+ *      mask_bits[px] set (one byte per pixel, NULL when n_masks == 0, masks may overlap).  Per class:
+ *        out_stats[class * 8 + 0..7] = mean, mae, rmse, min, max, median, medae, nmad;  out_count[class] = n
+ *      median = numpy's rule (even n: (a + b) / 2 of the two middle values); medae = median |r|;
+ *      nmad = 1.4826 * median |r - median(r)|.  count, min, max and the three medians are exact (MSD radix select on
+ *      order-preserving 64-bit codes, 8-bit digits, 16 passes over the rasters); the sums use a reduction tree fixed by
+ *      n, bitwise reproducible and independent of the other classes.  An empty class gives n = 0 and NaN elsewhere. */
+size_t t2h_residual_stats_workspace_bytes(int64_t n_px, int n_masks);
+int t2h_residual_stats(const double* pred, const double* gt, int64_t n_px, const uint8_t* mask_bits, int n_masks,
+                       int use_nodata, double nodata, void* workspace, size_t workspace_bytes, double* out_stats,
+                       int64_t* out_count, t2h_stream_t stream);
+
 /* bias gradient: out[c] = sum_r g[r, c], two-stage and deterministic */
 size_t t2h_colsum_workspace_bytes(int64_t rows, int n);
 int t2h_colsum(const float* g, int64_t ld_g, int64_t rows, int n, void* workspace,

@@ -14,6 +14,7 @@ from .topology import RaggedCloud  # noqa: F401
 from .adapters import load_config, ChunkCloud, write_raster, read_raster  # noqa: F401
 from .trainer import Trainer  # noqa: F401
 from .generator import SceneGenerator, OrthoImage  # noqa: F401
+from .evaluation import residual_stats  # noqa: F401
 
 
 def install_as_reference():

@@ -15,7 +15,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(_HERE)
 LIB_PATH = os.path.join(_HERE, "libt2h.so")
 CSRC = os.path.join(_HERE, "csrc")
-SOURCES = ["t2h_topology.cu", "t2h_segment.cu", "t2h_sample.cu", "t2h_scene.cu", "t2h_linear.cu", "t2h_blocks.cu"]
+SOURCES = ["t2h_topology.cu", "t2h_segment.cu", "t2h_sample.cu", "t2h_scene.cu", "t2h_linear.cu", "t2h_blocks.cu",
+           "t2h_eval.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 
@@ -48,6 +49,8 @@ SIGNATURES = {
     "t2h_tile_write": [_p, _p, _i64, _p, _f64, _f64, _p, _p, _p, _p],
     "t2h_blend_accumulate": [_p, _i32, _i32, _p, _p, _p, _p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p, _p],
     "t2h_raster_windows": [_p, _i32, _i64, _i64, _p, _p, _i32, _i32, _p, _p, _p, _p],
+    "t2h_residual_stats_workspace_bytes": [_i64, _i32],
+    "t2h_residual_stats": [_p, _p, _i64, _p, _i32, _i32, _f64, _p, _sz, _p, _p, _p],
     "t2h_upsample_bilinear_fwd": [_p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p],
     "t2h_upsample_bilinear_bwd": [_p, _i32, _i32, _i32, _i32, _i32, _i32, _p, _p],
     "t2h_split_tf32": [_p, _i64, _p, _p, _p],
@@ -80,7 +83,7 @@ _RESTYPE = {"t2h_status_string": ctypes.c_char_p, "t2h_sort_workspace_bytes": _s
             "t2h_linear_wgrad_workspace_bytes": _sz, "t2h_colsum_workspace_bytes": _sz,
             "t2h_conv3x3_wgrad_workspace_bytes": _sz, "t2h_bilinear_sample_bwd_workspace_bytes": _sz,
             "t2h_seg_workspace_bytes": _sz, "t2h_resblock_workspace_bytes": _sz,
-            "t2h_comm_mlp_workspace_bytes": _sz}
+            "t2h_comm_mlp_workspace_bytes": _sz, "t2h_residual_stats_workspace_bytes": _sz}
 
 _lib = None
 _lock = threading.Lock()

@@ -51,6 +51,18 @@ struct RowShape {
   static constexpr int C = 4 * LPR_ * CH_;
 };
 
+// order-preserving map double -> unsigned 64: a < b as doubles <=> encode_f64(a) < encode_f64(b) as integers (-0.0
+// sorts just below +0.0).  Integer atomicMin / atomicMax on the codes are deterministic; radix digits of the codes
+// select order statistics.
+__device__ __forceinline__ unsigned long long encode_f64(double v) {
+  const unsigned long long b = (unsigned long long)__double_as_longlong(v);
+  return (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double decode_f64(unsigned long long e) {
+  const unsigned long long b = (e & 0x8000000000000000ull) ? (e & 0x7fffffffffffffffull) : ~e;
+  return __longlong_as_double((long long)b);
+}
+
 __device__ __forceinline__ float4 ld4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 __device__ __forceinline__ void st4(float* p, const float4& v) { *reinterpret_cast<float4*>(p) = v; }
 // streaming variants: data touched once (do not keep it in L1)

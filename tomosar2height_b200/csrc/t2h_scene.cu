@@ -33,16 +33,6 @@ __device__ __forceinline__ bool first_crop(double x, double y, double x0, double
 }
 __device__ __forceinline__ bool second_crop(float nx, float ny) { return nx > 0.f && nx < 1.f && ny > 0.f && ny < 1.f; }
 
-// order-preserving map double -> unsigned 64 (for an integer atomicMin, which is deterministic)
-__device__ __forceinline__ unsigned long long encode_f64(double v) {
-  const unsigned long long b = (unsigned long long)__double_as_longlong(v);
-  return (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
-}
-__device__ __forceinline__ double decode_f64(unsigned long long e) {
-  const unsigned long long b = (e & 0x8000000000000000ull) ? (e & 0x7fffffffffffffffull) : ~e;
-  return __longlong_as_double((long long)b);
-}
-
 __global__ void __launch_bounds__(kCropThreads)
 tile_count_kernel(const double* __restrict__ pts, const CropItem* __restrict__ items, const double* __restrict__ tile_xy,
                   double patch, int32_t* __restrict__ item_count, unsigned long long* __restrict__ tile_zmin) {
