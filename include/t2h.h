@@ -178,8 +178,10 @@ int t2h_linear_fwd(const float* x1, int64_t ld_x1, int k1, const float* x2, int6
 /* 3xFP16 flavour of the same GEMM for wide layers (n_out > 64): kind::f16 tensor-core passes run at twice
  * the TF32 rate.  Both operands are scaled by a power of two taken from their maximum magnitude (scaled
  * maximum in [2^14, 2^15), exact), split into fp16 hi = rn(v), lo = rn(v - hi), multiplied as
- * lo*hi + hi*lo + hi*hi with fp32 accumulation and un-scaled in the epilogue: 2^-22 relative per product,
- * plus an absolute floor of 2^-40 of the operand maximum for entries that are tiny against it.
+ * lo*hi + hi*lo + hi*hi with fp32 accumulation and un-scaled in the epilogue: at most 3 x 2^-22 relative
+ * per product (the dropped lo*lo and the rounding of either lo, each <= 2^-22), plus an absolute floor of
+ * 2^-39 of the operand maximum for entries that are tiny against it (half the smallest fp16 subnormal
+ * against a scaled maximum >= 2^14; reached exactly, e.g. by an entry 2^-39 next to a maximum of 1).
  *   t2h_absmax:     *slot = bit pattern of max |[x1 | x2]| (x2 nullable / k2 = 0), pre-activation
  *   t2h_split_f16:  w (n fp32 values, n even) -> fp16 hi / lo under the scale of *absmax
  *   t2h_linear_fwd_f16: as t2h_linear_fwd with the fp16 weight split, (k1 + k2) % 8 == 0; out_absmax

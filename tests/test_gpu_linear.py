@@ -216,7 +216,7 @@ def test_linear_f16_operand_scaling(scale):
 
 def test_linear_f16_rows_of_very_different_magnitude():
     """rows spanning six orders of magnitude share one tensor scale: small rows keep ~1e-5 of THEIR OWN scale
-    (absolute floor 2^-40 of the tensor maximum, documented in include/t2h.h)."""
+    (absolute floor 2^-39 of the tensor maximum, documented in include/t2h.h)."""
     g = torch.Generator().manual_seed(12)
     x = torch.randn(4096, 256, generator=g) * torch.exp(torch.empty(4096, 1).uniform_(-12, 3, generator=g))
     w = torch.randn(256, 256, generator=g) / 16
