@@ -248,8 +248,11 @@ int t2h_conv3x3_wgrad_f16(const float* grad_out, const uint32_t* g_absmax, const
  * contiguous row ranges; `items`: work items of <= 1024 candidates, 16 bytes each {int32 tile, int32 count,
  * int64 first_row}; `tile_xy` (n_tiles, 2) float64 tile anchors (lower-left corner).
  *   t2h_tile_count: item_count[i] = survivors of both crops; tile_zmin[t] = order-preserving code of min z over the
- *                   first-crop survivors (initialise to all ones; an integer atomicMin, deterministic)
- *   t2h_tile_write: survivors as (x, y, z, 0) float32 rows in candidate order, item i starting at item_offset[i]
+ *                   first-crop survivors (initialise to all ones; an integer atomicMin, deterministic); a NaN z of
+ *                   either sign gives code 0 (z_shift NaN)
+ *   t2h_tile_write: survivors as (x, y, z, 0) float32 rows in candidate order, item i starting at item_offset[i];
+ *                   the items of a tile with code 0 write nothing (the reference drops such a tile), so the caller
+ *                   counts them as 0 in the scan
  *   t2h_blend_accumulate: for every raster pixel of the batch's bounding box, in tile order:
  *                   dsm += (double) heights[b, S-1-i, j] * wx[j] * wy[i];  weight += wx[j] * wy[i]            */
 int t2h_tile_count(const double* points, const void* items, int64_t n_items, const double* tile_xy, double patch,

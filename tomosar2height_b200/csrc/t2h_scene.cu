@@ -46,7 +46,9 @@ tile_count_kernel(const double* __restrict__ pts, const CropItem* __restrict__ i
     const double* p = pts + (it.first + i) * 3;
     const double x = p[0], y = p[1];
     if (first_crop(x, y, x0, y0, patch)) {
-      zmin = min(zmin, encode_f64(p[2]));
+      // NaN -> code 0, below every other code, so that one NaN z of either sign makes z_shift NaN like the reference's
+      // tile[:, 2].min() (encode_f64 alone puts a negative NaN below -inf but a positive one above +inf)
+      zmin = min(zmin, isnan(p[2]) ? 0ull : encode_f64(p[2]));
       cnt += second_crop((float)((x - x0) / patch), (float)((y - y0) / patch)) ? 1 : 0;
     }
   }
@@ -72,6 +74,9 @@ tile_write_kernel(const double* __restrict__ pts, const CropItem* __restrict__ i
   __shared__ int s_warp[kCropThreads / 32];
   __shared__ int s_base;
   const CropItem it = items[blockIdx.x];
+  // z_shift NaN (code 0): the reference's normalisation matrix, the inverse of a transform with a NaN translation, is
+  // NaN in every entry, so its re-crop drops every point of the tile.  The caller gives these items no rows.
+  if (tile_zmin[it.tile] == 0ull) return;
   const double x0 = tile_xy[2 * it.tile], y0 = tile_xy[2 * it.tile + 1];
   const double z_shift = decode_f64(tile_zmin[it.tile]);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;

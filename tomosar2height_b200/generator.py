@@ -201,9 +201,11 @@ class SceneGenerator:
         zmin = torch.full((n_tiles,), -1, dtype=torch.int64, device=dev)
         _lib.call("t2h_tile_count", _lib.ptr(binned), _lib.ptr(items_d), n_items, _lib.ptr(tile_xy), self.patch,
                   _lib.ptr(item_count), _lib.ptr(zmin))
-        counts64 = item_count.long()
+        item_tile = items_h[:, 0].to(dev)
+        # a tile with a NaN z (code 0) has no survivors, as in the reference: t2h_tile_write writes none of its rows
+        counts64 = item_count.long().masked_fill_(zmin[item_tile] == 0, 0)
         item_offset = (counts64.cumsum(0) - counts64).contiguous()
-        per_tile = torch.zeros(n_tiles, dtype=torch.int64, device=dev).index_add_(0, items_h[:, 0].to(dev), counts64)
+        per_tile = torch.zeros(n_tiles, dtype=torch.int64, device=dev).index_add_(0, item_tile, counts64)
         counts = per_tile.tolist()  # the one host read of the scene
         out = torch.empty(sum(counts), 4, dtype=torch.float32, device=dev)
         _lib.call("t2h_tile_write", _lib.ptr(binned), _lib.ptr(items_d), n_items, _lib.ptr(tile_xy), self.patch, self.z_scale,
